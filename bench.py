@@ -4,6 +4,7 @@
     python bench.py --gpus 1 --steps 20 --warmup 5
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
     python bench.py --impl reference ...        # the reference's CPU path (oracle port) on the host cores
+    python bench.py ... --dump-outputs DIR     # also write what the last timed step computed as DIR/<name>.npy
 
 A "step" = one pass of the hot path over one batch of 32 synthetic images: FAIDetr.forward (normalise -> ResNet50-vd ->
 hybrid encoder -> 6-layer deformable decoder) + the fused DETR post-process kernel.
@@ -36,6 +37,7 @@ METRIC = "images/sec fai-detr-l bs=32 640x640 inference"
 GFLOP_PER_IMG_USEFUL = 139.05  # SURVEY.md §8(d): excludes the dead mask_features conv
 IDEAL_US_PER_IMG_16BIT = 129.0  # SURVEY.md §8(d) sum-of-max roofline at 16-bit activations
 IDEAL_US_PER_IMG_FP32 = 259.0   # SURVEY.md §8(d): fp32 activations + half-rate (tf32-class) MMA
+DUMP_LIMIT_BYTES = 64 << 20
 
 
 def ncu_traffic(kernel_substr: str):
@@ -110,6 +112,23 @@ class ClockSampler:
                 if v.lower().startswith("active"):
                     reasons.add(name)
         return {"sm_mhz": float(np.median(sm)) if sm else None, "sm_max_mhz": max(mx) if mx else None, "reasons": sorted(reasons), "samples": len(sm)}
+
+
+def dump_outputs(path: str, arrays: dict) -> None:
+    """Write each tensor as <path>/<name>.npy: floating point as float32, integers as float64 (exact).  Smallest first; an array that would
+    take more than its share of what is left of DUMP_LIMIT_BYTES is replaced by a seeded sample of its flattened elements (the same
+    positions for the same shape), so two builds run with the same arguments write files that compare element for element."""
+    os.makedirs(path, exist_ok=True)
+    left = DUMP_LIMIT_BYTES
+    items = sorted(arrays.items(), key=lambda kv: kv[1].numel())
+    for i, (name, t) in enumerate(items):
+        a = t.detach().float().cpu().numpy() if t.is_floating_point() else t.detach().cpu().numpy().astype(np.float64)
+        share = left // (len(items) - i)
+        if a.nbytes > share:
+            idx = np.sort(np.random.default_rng(0).choice(a.size, share // a.itemsize, replace=False))
+            a = a.reshape(-1)[idx]
+        np.save(os.path.join(path, name + ".npy"), a)
+        left -= a.nbytes
 
 
 def cpu_reference_run(batch: int, steps: int, warmup: int, sd, threads: int):
@@ -194,7 +213,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--quick", action="store_true", help="skip the bs=1 latency, parity-mode and other-config legs")
     ap.add_argument("--no-other-configs", action="store_true", help="skip the MaskFormer / BisenetFormer / fine-tune legs (separate processes)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last one computed (model logits / boxes and the "
+                    "post-processed detections of rank 0) as DIR/<name>.npy, at most 64 MB in all")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the CUDA path (--impl ours)")
     rank = int(os.environ.get("RANK", 0))
     local_rank = int(os.environ.get("LOCAL_RANK", 0))
     world = int(os.environ.get("WORLD_SIZE", 1))
@@ -240,7 +265,7 @@ def main():
 
     def step_device():
         out = fm.model(x_dev)
-        return ops.detr_postprocess(out.logits, out.boxes, sizes_dev, 300, 0.5)
+        return out, ops.detr_postprocess(out.logits, out.boxes, sizes_dev, 300, 0.5)
 
     # ---- warm-up (also builds the engine), then capture forward+post-process in a CUDA graph
     l0 = ops.launch_count()
@@ -263,8 +288,8 @@ def main():
     def run_step():
         if graph is not None:
             graph.replay()
-        else:
-            step_device()
+            return g_out
+        return step_device()
 
     for _ in range(max(args.warmup, 3)):
         run_step()
@@ -276,9 +301,13 @@ def main():
     with ClockSampler(local_rank) as clk:
         e0.record()
         for _ in range(args.steps):
-            run_step()
+            last = run_step()
         e1.record()
         torch.cuda.synchronize()
+    if args.dump_outputs and rank == 0:
+        out, (d_scores, d_labels, d_boxes, d_query, d_count) = last
+        dump_outputs(args.dump_outputs, {"logits": out.logits, "boxes": out.boxes, "det_scores": d_scores, "det_labels": d_labels,
+                                         "det_boxes": d_boxes, "det_query": d_query, "det_count": d_count})
     ms_total = D.max_over_ranks(e0.elapsed_time(e1), dev)  # device time, max over ranks
     D.synchronize()
     ms_step = ms_total / args.steps

@@ -9,17 +9,13 @@ if ROOT not in sys.path:
 
 
 def pytest_configure(config):
-    config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 box with -m gpu)")
-    config.addinivalue_line("markers", "reference: needs the read-only reference tree at /root/reference (build container only)")
+    config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 with -m gpu)")
 
 
 def pytest_collection_modifyitems(config, items):
     import torch
 
     has_gpu = torch.cuda.is_available()
-    has_ref = os.path.isdir("/root/reference/focoos")
     for it in items:
         if "gpu" in it.keywords and not has_gpu:
             it.add_marker(pytest.mark.skip(reason="no CUDA device"))
-        if "reference" in it.keywords and not has_ref:
-            it.add_marker(pytest.mark.skip(reason="/root/reference not present"))

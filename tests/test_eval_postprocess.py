@@ -1,13 +1,18 @@
-"""DETRProcessor.eval_postprocess (SURVEY §8 f3): host logic on the CPU reference backend against the UNMODIFIED reference's
-`DETRProcessor.eval_postprocess` (build container only), and the CUDA kernel against the CPU reference operator (-m gpu)."""
+"""DETRProcessor.eval_postprocess (SURVEY §8 f3): host logic on the CPU reference backend against what the UNMODIFIED reference's
+`DETRProcessor.eval_postprocess` returns for the same case (tests/golden/reference_checks.json, oracle/gen_golden_reference_checks.py),
+and the CUDA kernel against the CPU reference operator (-m gpu)."""
+import json
+import os
+
 import numpy as np
 import pytest
 import torch
 
 from focoos_b200 import DETRConfig, DETRProcessor, ops
 from focoos_b200.ports import DETRModelOutput
-from oracle import ref_import
 from oracle.ops_ref import RefBackend
+
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_checks.json")
 
 
 def _case(B=3, Q=300, C=20, seed=0):
@@ -39,23 +44,14 @@ def _check_against(res, ref_scores, ref_labels, ref_boxes):
         assert np.abs(inst.boxes.tensor.cpu().numpy() - b).max() <= 1e-4 if len(s) else True
 
 
-@pytest.mark.reference
 def test_eval_postprocess_matches_the_reference(ref_backend):
-    ref_import.install()
-    from focoos.models.fai_detr.config import DETRConfig as RC
-    from focoos.models.fai_detr.ports import DETRModelOutput as RO
-    from focoos.models.fai_detr.processor import DETRProcessor as RP
-
-    class Entry:  # DatasetEntry duck type
-        def __init__(self, d):
-            self.height, self.width = d["height"], d["width"]
-
+    with open(GOLDEN) as f:
+        ref = json.load(f)["eval_postprocess"]
     logits, boxes, entries = _case()
-    from focoos.nn.backbone.resnet import ResnetConfig as RB
-    ref = RP(RC(backbone_config=RB(), num_classes=20), image_size=640).eval_postprocess(RO(boxes=boxes.clone(), logits=logits.clone(), loss=None), [Entry(e) for e in entries], top_k=100)
     ours = DETRProcessor(DETRConfig(num_classes=20), image_size=640).eval_postprocess(DETRModelOutput(boxes=boxes, logits=logits), entries, top_k=100)
-    _check_against(ours, [r["instances"].scores.numpy() for r in ref], [r["instances"].classes.numpy() for r in ref], [r["instances"].boxes.tensor.numpy() for r in ref])
-    assert [o["instances"].image_size for o in ours] == [tuple(r["instances"].image_size) for r in ref]
+    _check_against(ours, [np.array(r["scores"], dtype=np.float32) for r in ref], [np.array(r["classes"], dtype=np.int64) for r in ref],
+                   [np.array(r["boxes"], dtype=np.float32).reshape(-1, 4) for r in ref])
+    assert [o["instances"].image_size for o in ours] == [tuple(r["image_size"]) for r in ref]
 
 
 @pytest.mark.gpu

@@ -1,6 +1,6 @@
 """The PNG / base64 tail of the segmentation post-process (SURVEY §8 a17 / f2; reference utils/vision.py:264-293, pinned in the reference by
-tests/utils/test_vision.py:154-160): byte-identical strings to the unmodified reference function (goldens from oracle/gen_golden_png.py),
-and the decoded image is the mask."""
+tests/utils/test_vision.py:154-160): byte-identical strings to the unmodified reference function (goldens from oracle/gen_golden_png.py and
+oracle/gen_golden_reference_checks.py), and the decoded image is the mask."""
 import json
 import os
 
@@ -8,9 +8,10 @@ import numpy as np
 import pytest
 
 from focoos_b200.processor import base64_to_binary_mask, binary_mask_to_base64
-from oracle import ref_import
+from oracle.gen_golden_reference_checks import png_masks
 
 GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "png_masks.json")
+REFERENCE_CHECKS = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_checks.json")
 
 
 def _cases():
@@ -36,14 +37,12 @@ def test_reference_fixture_mask():
     assert isinstance(s, str) and np.array_equal(base64_to_binary_mask(s), m)
 
 
-@pytest.mark.reference
 def test_against_the_live_reference_function():
-    ref_import.install()
-    import cv2
-    if type(cv2).__name__.startswith("_Dummy"):
-        pytest.skip("OpenCV absent")
-    from focoos.utils.vision import binary_mask_to_base64 as ref_fn
-    rng = np.random.default_rng(11)
-    for shape in ((1, 1), (5, 7), (120, 33), (64, 64)):
-        m = rng.random(shape) > 0.6
-        assert binary_mask_to_base64(m) == ref_fn(m)
+    """seeded random masks of several shapes -> the strings the reference function returned for them"""
+    pytest.importorskip("cv2")
+    with open(REFERENCE_CHECKS) as f:
+        ref = json.load(f)["png_b64"]
+    masks = png_masks()
+    assert len(masks) == len(ref)
+    for shape, m in masks:
+        assert binary_mask_to_base64(m) == ref["x".join(map(str, shape))]
