@@ -20,175 +20,11 @@ training (torch.autocast(fp16) + GradScaler, trainer/trainer.py:645,735-771), a 
 """
 from __future__ import annotations
 
-import ctypes
 from typing import Optional, Sequence, Tuple
 
 import torch
 
 from . import ops
-from .ops import CudaBackend, _p, _stream
-
-ops.EXPORTED_SYMBOLS = ops.EXPORTED_SYMBOLS + (
-    "fb200_conv_wgrad_workspace_bytes", "fb200_conv_wgrad", "fb200_conv_wgrad_tc_supported", "fb200_conv_wgrad_tc_workspace_bytes", "fb200_conv_wgrad_tc", "fb200_conv_wgrad_tc_f16", "fb200_dilate2", "fb200_col_workspace_bytes", "fb200_colsum", "fb200_bn_train_fwd", "fb200_bn_train_bwd", "fb200_bn_stats", "fb200_bn_sync_combine", "fb200_bn_apply", "fb200_bn_bwd_reduce", "fb200_bn_bwd_apply",
-    "fb200_add_act", "fb200_maxpool3x3s2_bwd", "fb200_avgpool2x2_ceil_bwd", "fb200_resize_bilinear_bwd", "fb200_layernorm_bwd", "fb200_attention_bwd", "fb200_msda_bwd")
-
-_f = ctypes.c_float
-
-
-def _ws(nbytes: int, device):
-    return torch.empty(int(nbytes), dtype=torch.uint8, device=device)
-
-
-# ---- backend methods (mirrored on oracle.ops_ref.RefBackend for the CPU host-logic tests) ---------------------------
-def _cb_conv_wgrad(self, x, dy, KH, KW, stride, pad, dw):
-    self._cuda(x, dy, dw)
-    B, H, W, Cin = x.shape
-    _, Ho, Wo, Cout = dy.shape
-    self.lib.fb200_conv_wgrad_workspace_bytes.restype = ctypes.c_int64
-    ws = _ws(self.lib.fb200_conv_wgrad_workspace_bytes(B, Ho, Wo, Cin, Cout, KH, KW), x.device)
-    self._call("fb200_conv_wgrad", _p(x), B, H, W, Cin, x.stride(2), _p(dy), Ho, Wo, Cout, dy.stride(2), KH, KW, stride, pad, _p(dw), 0, _p(ws), _stream())
-
-
-def _cb_conv_wgrad_tc_supported(self, x_shape, dy_shape, KH, KW, stride, pad):
-    B, H, W, Cin = x_shape
-    _, Ho, Wo, Cout = dy_shape
-    return bool(self.lib.fb200_conv_wgrad_tc_supported(B, H, W, Cin, Ho, Wo, Cout, KH, KW, stride, pad))
-
-
-def _cb_conv_wgrad_tc(self, x_pair, dy_pair, KH, KW, stride, pad, dw):
-    self._cuda(x_pair, dy_pair, dw)
-    B, H, W, C2 = x_pair.shape
-    Cin, Cout = C2 // 2, dy_pair.shape[-1] // 2
-    self.lib.fb200_conv_wgrad_tc_workspace_bytes.restype = ctypes.c_int64
-    ws = _ws(self.lib.fb200_conv_wgrad_tc_workspace_bytes(B, dy_pair.shape[1], dy_pair.shape[2], Cin, Cout, KH, KW), x_pair.device)
-    self._call("fb200_conv_wgrad_tc", _p(x_pair), B, H, W, Cin, _p(dy_pair), Cout, KH, KW, stride, pad, _p(dw), 0, _p(ws), _stream())
-
-
-def _cb_conv_wgrad_tc_f16(self, x16, dy16, KH, KW, stride, pad, dw):
-    self._cuda(x16, dy16, dw)
-    B, H, W, Cin = x16.shape
-    Cout = dy16.shape[-1]
-    self.lib.fb200_conv_wgrad_tc_workspace_bytes.restype = ctypes.c_int64
-    ws = _ws(self.lib.fb200_conv_wgrad_tc_workspace_bytes(B, dy16.shape[1], dy16.shape[2], Cin, Cout, KH, KW), x16.device)
-    self._call("fb200_conv_wgrad_tc_f16", _p(x16), B, H, W, Cin, _p(dy16), Cout, KH, KW, stride, pad, _p(dw), 0, _p(ws), _stream())
-
-
-def _cb_dilate2(self, dy, out):
-    self._cuda(dy, out)
-    B, Ho, Wo, C = dy.shape
-    self._call("fb200_dilate2", _p(dy), B, Ho, Wo, C, out.shape[1], out.shape[2], _p(out), _stream())
-
-
-def _col_ws(self, C, device):
-    self.lib.fb200_col_workspace_bytes.restype = ctypes.c_int64
-    return _ws(self.lib.fb200_col_workspace_bytes(C), device)
-
-
-def _cb_colsum(self, x2d, out):
-    self._cuda(x2d, out)
-    R, C = x2d.shape
-    self._call("fb200_colsum", _p(x2d), ctypes.c_int64(R), C, x2d.stride(0), _p(out), 0, _p(_col_ws(self, C, x2d.device)), _stream())
-
-
-def _cb_bn_train_fwd(self, x2d, gamma, beta, res2d, act, eps, momentum, rmean, rvar, save_mean, save_rstd, y2d):
-    self._cuda(x2d, gamma, beta, y2d)
-    R, C = x2d.shape
-    self._call("fb200_bn_train_fwd", _p(x2d), x2d.stride(0), ctypes.c_int64(R), C, _p(gamma), _p(beta), _p(res2d), 0 if res2d is None else res2d.stride(0), act, _f(eps),
-               _f(momentum), _p(rmean), _p(rvar), _p(save_mean), _p(save_rstd), _p(y2d), y2d.stride(0), _p(_col_ws(self, C, x2d.device)), _stream())
-
-
-def _cb_bn_train_bwd(self, x2d, dy2d, y2d, gamma, beta, save_mean, save_rstd, act, dx2d, dres2d, dgamma, dbeta):
-    self._cuda(x2d, dy2d, dx2d)
-    R, C = x2d.shape
-    self._call("fb200_bn_train_bwd", _p(x2d), x2d.stride(0), _p(dy2d), dy2d.stride(0), _p(y2d), 0 if y2d is None else y2d.stride(0), ctypes.c_int64(R), C, _p(gamma), _p(beta),
-               _p(save_mean), _p(save_rstd), act, _p(dx2d), dx2d.stride(0), _p(dres2d), 0 if dres2d is None else dres2d.stride(0), _p(dgamma), _p(dbeta), 0,
-               _p(_col_ws(self, C, x2d.device)), _stream())
-
-
-def _cb_bn_stats(self, x2d, mean, var):
-    self._cuda(x2d, mean, var)
-    R, C = x2d.shape
-    self._call("fb200_bn_stats", _p(x2d), x2d.stride(0), ctypes.c_int64(R), C, _p(mean), _p(var), _p(_col_ws(self, C, x2d.device)), _stream())
-
-
-def _cb_bn_sync_combine(self, allst, eps, momentum, rmean, rvar, mean, rstd, inv_total):
-    self._cuda(allst, mean, rstd, inv_total)
-    world, width = allst.shape
-    self._call("fb200_bn_sync_combine", _p(allst), world, (width - 1) // 2, _f(eps), _f(momentum), _p(rmean), _p(rvar), _p(mean), _p(rstd), _p(inv_total), _stream())
-
-
-def _cb_bn_apply(self, x2d, mean, rstd, gamma, beta, res2d, act, y2d):
-    self._cuda(x2d, mean, rstd, gamma, beta, y2d)
-    R, C = x2d.shape
-    self._call("fb200_bn_apply", _p(x2d), x2d.stride(0), ctypes.c_int64(R), C, _p(mean), _p(rstd), _p(gamma), _p(beta), _p(res2d), 0 if res2d is None else res2d.stride(0), act,
-               _p(y2d), y2d.stride(0), _stream())
-
-
-def _cb_bn_bwd_reduce(self, x2d, dy2d, y2d, gamma, beta, mean, rstd, act, sum_dy, sum_dy_xhat):
-    self._cuda(x2d, dy2d, sum_dy, sum_dy_xhat)
-    R, C = x2d.shape
-    self._call("fb200_bn_bwd_reduce", _p(x2d), x2d.stride(0), _p(dy2d), dy2d.stride(0), _p(y2d), 0 if y2d is None else y2d.stride(0), ctypes.c_int64(R), C, _p(gamma), _p(beta),
-               _p(mean), _p(rstd), act, _p(sum_dy), _p(sum_dy_xhat), _p(_col_ws(self, C, x2d.device)), _stream())
-
-
-def _cb_bn_bwd_apply(self, x2d, dy2d, y2d, gamma, beta, mean, rstd, sum_dy, sum_dy_xhat, inv_count, act, dx2d, dres2d):
-    self._cuda(x2d, dy2d, dx2d)
-    R, C = x2d.shape
-    self._call("fb200_bn_bwd_apply", _p(x2d), x2d.stride(0), _p(dy2d), dy2d.stride(0), _p(y2d), 0 if y2d is None else y2d.stride(0), ctypes.c_int64(R), C, _p(gamma), _p(beta),
-               _p(mean), _p(rstd), _p(sum_dy), _p(sum_dy_xhat), _f(inv_count), act, _p(dx2d), dx2d.stride(0), _p(dres2d), 0 if dres2d is None else dres2d.stride(0), _stream())
-
-
-def _cb_add_act(self, a, b, dy, act, out):
-    self._cuda(a, out)
-    self._call("fb200_add_act", _p(a), _p(b), _p(dy), act, ctypes.c_int64(a.numel()), _p(out), _stream())
-
-
-def _cb_maxpool_bwd(self, x, dy, dx):
-    self._cuda(x, dy, dx)
-    B, H, W, C = x.shape
-    self._call("fb200_maxpool3x3s2_bwd", _p(x), _p(dy), B, H, W, C, _p(dx), _stream())
-
-
-def _cb_avgpool_bwd(self, dy, dx):
-    self._cuda(dy, dx)
-    B, H, W, C = dx.shape
-    self._call("fb200_avgpool2x2_ceil_bwd", _p(dy), B, H, W, C, _p(dx), _stream())
-
-
-def _cb_resize_bwd(self, dy, dx):
-    self._cuda(dy, dx)
-    B, H, W, C = dx.shape
-    self._call("fb200_resize_bilinear_bwd", _p(dy), dy.stride(2), B, H, W, C, dy.shape[1], dy.shape[2], _p(dx), _stream())
-
-
-def _cb_layernorm_bwd(self, x2d, res2d, gamma, dy2d, eps, dx2d, dgamma, dbeta):
-    self._cuda(x2d, dy2d, dx2d)
-    M, C = x2d.shape
-    self._call("fb200_layernorm_bwd", _p(x2d), _p(res2d), _p(gamma), _p(dy2d), ctypes.c_int64(M), C, _f(eps), _p(dx2d), _p(dgamma), _p(dbeta), 0,
-               _p(_col_ws(self, C, x2d.device)), _stream())
-
-
-def _cb_attention_bwd(self, q, k, v, o, do, heads, scale, dq, dk, dv):
-    self._cuda(q, k, v, o, do, dq, dk, dv)
-    B, Lq, C = q.shape
-    self._call("fb200_attention_bwd", _p(q), q.stride(1), _p(k), k.stride(1), _p(v), v.stride(1), _p(o), o.stride(1), _p(do), do.stride(1), B, Lq, k.shape[1], heads,
-               C // heads, _f(scale), _p(dq), dq.stride(1), _p(dk), dk.stride(1), _p(dv), dv.stride(1), _stream())
-
-
-def _cb_msda_bwd(self, value, oa, ref, do, shapes, P, heads, dvalue, doa):
-    self._cuda(value, oa, ref, do, dvalue, doa)
-    B, S, _ = value.shape
-    Q = oa.shape[1]
-    arr = (ctypes.c_int * (2 * len(shapes)))(*[int(v) for hw in shapes for v in hw])
-    self._call("fb200_msda_bwd", _p(value), value.stride(1), _p(oa), oa.stride(1), _p(ref), _p(do), do.stride(1), arr, len(shapes), P, B, S, Q, heads, _p(dvalue),
-               dvalue.stride(1), _p(doa), doa.stride(1), _stream())
-
-
-for _n, _fn in (("conv_wgrad", _cb_conv_wgrad), ("conv_wgrad_tc_supported", _cb_conv_wgrad_tc_supported), ("conv_wgrad_tc", _cb_conv_wgrad_tc), ("conv_wgrad_tc_f16", _cb_conv_wgrad_tc_f16), ("dilate2", _cb_dilate2), ("colsum", _cb_colsum), ("bn_train_fwd", _cb_bn_train_fwd), ("bn_train_bwd", _cb_bn_train_bwd),
-                ("bn_stats", _cb_bn_stats), ("bn_sync_combine", _cb_bn_sync_combine), ("bn_apply", _cb_bn_apply), ("bn_bwd_reduce", _cb_bn_bwd_reduce), ("bn_bwd_apply", _cb_bn_bwd_apply),
-                ("add_act", _cb_add_act), ("maxpool_bwd", _cb_maxpool_bwd), ("avgpool_bwd", _cb_avgpool_bwd), ("resize_bwd", _cb_resize_bwd),
-                ("layernorm_bwd", _cb_layernorm_bwd), ("attention_bwd", _cb_attention_bwd), ("msda_bwd", _cb_msda_bwd)):
-    setattr(CudaBackend, _n, _fn)
 
 
 # ---- conv through either fp32 engine ----------------------------------------------------------------------------------

@@ -10,50 +10,18 @@ torch.autograd.Function hands back to whatever produced the predictions.  No CPU
 """
 from __future__ import annotations
 
-import ctypes
 from dataclasses import dataclass
 from typing import Dict, List, Sequence, Tuple
 
 import torch
 
 from . import ops
-from .ops import CudaBackend, _p, _stream
-
-ops.EXPORTED_SYMBOLS = ops.EXPORTED_SYMBOLS + ("fb200_detr_match_cost", "fb200_hungarian", "fb200_detr_loss_workspace_bytes", "fb200_detr_loss")
 
 
 @dataclass
 class DETRTargets:
     labels: torch.Tensor  # [n] int64 class ids
     boxes: torch.Tensor   # [n,4] cxcywh normalised to [0,1]
-
-
-# ---- backend methods (same names on oracle.ops_ref.RefBackend for the CPU host-logic tests) -------------------
-def _cb_detr_match_cost(self, logits, boxes, tl, tb, toff, wts, alpha, gamma, cost):
-    self._cuda(logits, boxes, tl, tb, toff, cost)
-    L, B, Q, C = logits.shape
-    self._call("fb200_detr_match_cost", _p(logits), _p(boxes), _p(tl), _p(tb), _p(toff), L, B, Q, C, tl.shape[0],
-               ctypes.c_float(wts[0]), ctypes.c_float(wts[1]), ctypes.c_float(wts[2]), ctypes.c_float(alpha), ctypes.c_float(gamma), _p(cost), _stream())
-
-
-def _cb_hungarian(self, cost, toff, B, max_targets, match_q):
-    self._cuda(cost, toff, match_q)
-    L, T, Q = cost.shape
-    self._call("fb200_hungarian", _p(cost), _p(toff), L, B, Q, T, max_targets, _p(match_q), _stream())
-
-
-def _cb_detr_loss(self, logits, boxes, tl, tb, toff, match_q, num_boxes, wts, alpha, gamma, losses, g_logits, g_l1, g_giou):
-    self._cuda(logits, boxes, toff, losses, g_logits, g_l1, g_giou)
-    L, B, Q, C = logits.shape
-    self.lib.fb200_detr_loss_workspace_bytes.restype = ctypes.c_int64
-    ws = torch.empty(int(self.lib.fb200_detr_loss_workspace_bytes(L, B, Q)), dtype=torch.uint8, device=logits.device)
-    self._call("fb200_detr_loss", _p(logits), _p(boxes), _p(tl), _p(tb), _p(toff), _p(match_q), L, B, Q, C, 0 if tl is None else tl.shape[0],
-               ctypes.c_float(num_boxes), ctypes.c_float(wts[0]), ctypes.c_float(wts[1]), ctypes.c_float(wts[2]), ctypes.c_float(alpha), ctypes.c_float(gamma),
-               _p(losses), _p(g_logits), _p(g_l1), _p(g_giou), _p(ws), _stream())
-
-
-for _n, _f in (("detr_match_cost", _cb_detr_match_cost), ("hungarian", _cb_hungarian), ("detr_loss", _cb_detr_loss)):
-    setattr(CudaBackend, _n, _f)
 
 
 def _pack_targets(targets: Sequence[DETRTargets], device):

@@ -17,6 +17,7 @@ from __future__ import annotations
 
 import ctypes
 import os
+import re
 from typing import Optional, Sequence, Tuple
 
 import numpy as np
@@ -44,8 +45,36 @@ def torch_dtype(code: int) -> torch.dtype:
     return torch.float32 if code == F32 else torch.float16
 
 
+_HEADER = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "include", "focoos_b200.h")
+_RESTYPES = {"int": ctypes.c_int, "int64_t": ctypes.c_int64, "const char*": ctypes.c_char_p}
+_ARGTYPES = {"int": ctypes.c_int, "int64_t": ctypes.c_int64, "float": ctypes.c_float}  # and every pointer: c_void_p
+
+
+def _ctype(table, decl: str, fn: str):
+    if decl in table:
+        return table[decl]
+    if table is _ARGTYPES and "*" in decl:
+        return ctypes.c_void_p
+    raise RuntimeError(f"focoos_b200: {fn} in {_HEADER} uses the type `{decl}`, which the ctypes binding does not map")
+
+
+def _prototypes():
+    """{name: (restype, argtypes)} of every `ret fb200_name(params);` declared in include/focoos_b200.h"""
+    text = re.sub(r"/\*.*?\*/", "", open(_HEADER).read(), flags=re.S)
+    protos = {}
+    for ret, name, params in re.findall(r"^\s*([\w ]+\**)\s*\b(fb200_\w+)\s*\(([^)]*)\)\s*;", text, flags=re.M):
+        params = [] if params.strip() in ("", "void") else [re.sub(r"\s*\b\w+$", "", p.strip()) for p in params.split(",")]
+        protos[name] = (_ctype(_RESTYPES, ret.strip(), name), [_ctype(_ARGTYPES, p, name) for p in params])
+    return protos
+
+
+_PROTOTYPES = _prototypes()
+EXPORTED_SYMBOLS = tuple(sorted(_PROTOTYPES))
+
+
 def load_library():
-    """Load the C-ABI library; raises if it has not been built (no silent fallback)."""
+    """Load the C-ABI library with the prototypes of include/focoos_b200.h; raises if it has not been built (no silent fallback)
+    or does not export a declared entry point."""
     global _lib
     if _lib is not None:
         return _lib
@@ -55,22 +84,11 @@ def load_library():
             "`python -m focoos_b200.csrc.build` (or `__graft_entry__.build()`); there is no CPU fallback."
         )
     lib = ctypes.CDLL(_LIB_PATH)
-    lib.fb200_last_error.restype = ctypes.c_char_p
-    for name in EXPORTED_SYMBOLS:
-        if name != "fb200_last_error":
-            getattr(lib, name).restype = ctypes.c_int
+    for name, (restype, argtypes) in _PROTOTYPES.items():
+        fn = getattr(lib, name)
+        fn.restype, fn.argtypes = restype, argtypes
     _lib = lib
     return lib
-
-
-EXPORTED_SYMBOLS = (
-    "fb200_last_error", "fb200_version", "fb200_device_supports_tcgen05", "fb200_set_option", "fb200_set_conv_trace", "fb200_stem_conv3x3s2", "fb200_stem_conv3x3s2_u8", "fb200_conv2d", "fb200_conv2d_per_image_weights", "fb200_linear_rowmax", "fb200_image_resize",
-    "fb200_split_f32_pair", "fb200_conv2d_pair", "fb200_pair_pool", "fb200_linear_rowmax_pair",
-    "fb200_maxpool3x3s2", "fb200_avgpool2x2_ceil", "fb200_resize_bilinear", "fb200_add", "fb200_layernorm",
-    "fb200_attention", "fb200_attention_split", "fb200_msda", "fb200_row_select", "fb200_rowmax", "fb200_topk", "fb200_gather_rows",
-    "fb200_box_op", "fb200_detr_postprocess", "fb200_detr_eval_postprocess",
-    "fb200_layernorm_ex", "fb200_split_pair_ex", "fb200_box_refine_qpos", "fb200_sigmoid_rows",
-)
 
 _launch_count = 0
 _trace = None       # profiling aid (tools/layer_roofline.py): list of [symbol, note, start_event, end_event]
@@ -95,11 +113,15 @@ def _check(rc: int, what: str):
 
 
 def _p(t: Optional[torch.Tensor]):
-    return ctypes.c_void_p(0 if t is None else t.data_ptr())
+    return None if t is None else t.data_ptr()
 
 
 def _stream():
-    return ctypes.c_void_p(torch.cuda.current_stream().cuda_stream)
+    return torch.cuda.current_stream().cuda_stream
+
+
+def _ws(nbytes: int, device):
+    return torch.empty(int(nbytes), dtype=torch.uint8, device=device)
 
 
 def _pitch(t: torch.Tensor, free_batch_stride: bool = False) -> int:
@@ -161,18 +183,18 @@ class CudaBackend:
         if _trace is not None:
             _trace_note.append(dict(op="conv", B=B, H=H, W=W, Cin=Cin, Cout=Cout, k=KH, stride=stride, res=residual is not None, xdt=str(x.dtype)[6:], odt=str(out.dtype)[6:], algo=algo))
         self._call("fb200_conv2d", _p(x), _dt(x), B, H, W, Cin, _pitch(x), _p(w), KH, KW, stride, pad, _p(scale), _p(bias), _p(residual),
-                   0 if residual is None else _pitch(residual), act, _p(out), _dt(out), _pitch(out, True), ctypes.c_int64(_batch_stride(out)), Cout, algo, _stream())
+                   0 if residual is None else _pitch(residual), act, _p(out), _dt(out), _pitch(out, True), _batch_stride(out), Cout, algo, _stream())
 
     def conv2d_per_image(self, x, w, act, out, algo):
         self._cuda(x, w, out)
         B, H, W, Cin = x.shape
         _, Cout, KH, KW, _ = w.shape
-        self._call("fb200_conv2d_per_image_weights", _p(x), _dt(x), B, H, W, Cin, _pitch(x), _p(w), ctypes.c_int64(w.stride(0)), KH, KW, 1, (KH - 1) // 2, None, None, act,
+        self._call("fb200_conv2d_per_image_weights", _p(x), _dt(x), B, H, W, Cin, _pitch(x), _p(w), w.stride(0), KH, KW, 1, (KH - 1) // 2, None, None, act,
                    _p(out), _dt(out), _pitch(out, True), Cout, algo, _stream())
 
     def linear_rowmax(self, x2d, w, bias, out):
         self._cuda(x2d, w, out)
-        self._call("fb200_linear_rowmax", _p(x2d), ctypes.c_int64(x2d.shape[0]), x2d.shape[1], x2d.stride(0), _p(w), _p(bias), w.shape[0], _p(out), _stream())
+        self._call("fb200_linear_rowmax", _p(x2d), x2d.shape[0], x2d.shape[1], x2d.stride(0), _p(w), _p(bias), w.shape[0], _p(out), _stream())
 
     def conv2d_pair(self, x, w3, scale, bias, stride, pad, act, residual, out):
         """x / residual / out: `Pair` (hi + lo fp16 planes) - residual and out may also be plain fp32 tensors (both, or neither)"""
@@ -185,9 +207,9 @@ class CudaBackend:
         rh = None if residual is None else (residual.hi if out_pair else residual)
         if _trace is not None:
             _trace_note.append(dict(op="conv", B=B, H=H, W=W, Cin=C, Cout=Cout, k=KH, stride=stride, res=residual is not None, xdt="pair", odt="pair" if out_pair else "float32", algo=3))
-        self._call("fb200_conv2d_pair", _p(xh), B, H, W, C, _pitch(xh), ctypes.c_int64(x.lo_off), _p(w3), KH, KW, stride, pad, _p(scale), _p(bias), _p(rh),
-                   0 if rh is None else _pitch(rh), ctypes.c_int64(residual.lo_off if (out_pair and residual is not None) else 0), act, _p(oh), F16PAIR if out_pair else F32,
-                   _pitch(oh, True), ctypes.c_int64(out.lo_off if out_pair else 0), ctypes.c_int64(_batch_stride(oh)), Cout, _stream())
+        self._call("fb200_conv2d_pair", _p(xh), B, H, W, C, _pitch(xh), x.lo_off, _p(w3), KH, KW, stride, pad, _p(scale), _p(bias), _p(rh),
+                   0 if rh is None else _pitch(rh), residual.lo_off if (out_pair and residual is not None) else 0, act, _p(oh), F16PAIR if out_pair else F32,
+                   _pitch(oh, True), out.lo_off if out_pair else 0, _batch_stride(oh), Cout, _stream())
 
     def image_resize(self, images, out):
         self._cuda(images, out)
@@ -200,18 +222,18 @@ class CudaBackend:
         xh, oh = x.hi, out.hi
         self._cuda(xh, oh)
         B, H, W, C = xh.shape
-        self._call("fb200_pair_pool", mode, _p(xh), ctypes.c_int64(x.lo_off), _pitch(xh), B, H, W, C, _p(oh), ctypes.c_int64(out.lo_off), _pitch(oh), oh.shape[1], oh.shape[2], _stream())
+        self._call("fb200_pair_pool", mode, _p(xh), x.lo_off, _pitch(xh), B, H, W, C, _p(oh), out.lo_off, _pitch(oh), oh.shape[1], oh.shape[2], _stream())
 
     def linear_rowmax_pair(self, xp, w3, bias, out):
         xh = xp.hi
         self._cuda(xh, w3, out)
         M = xh.numel() // xh.shape[-1]
-        self._call("fb200_linear_rowmax_pair", _p(xh), ctypes.c_int64(M), xh.shape[-1], _pitch(xh), ctypes.c_int64(xp.lo_off), _p(w3), _p(bias), w3.shape[0], _p(out), _stream())
+        self._call("fb200_linear_rowmax_pair", _p(xh), M, xh.shape[-1], _pitch(xh), xp.lo_off, _p(w3), _p(bias), w3.shape[0], _p(out), _stream())
 
     def split_pair(self, x, out):
         self._cuda(x, out)
         C = x.shape[-1]
-        self._call("fb200_split_f32_pair", _p(x), ctypes.c_int64(x.numel() // C), C, _pitch(x), _p(out), _stream())
+        self._call("fb200_split_f32_pair", _p(x), x.numel() // C, C, _pitch(x), _p(out), _stream())
 
     def maxpool3x3s2(self, x, out):
         self._cuda(x, out)
@@ -231,12 +253,12 @@ class CudaBackend:
     def add(self, a, b, out):
         self._cuda(a, b, out)
         C = a.shape[-1]
-        self._call("fb200_add", _p(a), _p(b), _p(out), _dt(a), ctypes.c_int64(a.numel() // C), ctypes.c_int64(b.numel() // C), C, _stream())
+        self._call("fb200_add", _p(a), _p(b), _p(out), _dt(a), a.numel() // C, b.numel() // C, C, _stream())
 
     def layernorm(self, x, res, gamma, beta, out, eps):
         self._cuda(x, out)
         C = x.shape[-1]
-        self._call("fb200_layernorm", _p(x), _p(res), _p(gamma), _p(beta), _p(out), _dt(x), ctypes.c_int64(x.numel() // C), C, ctypes.c_float(eps), _stream())
+        self._call("fb200_layernorm", _p(x), _p(res), _p(gamma), _p(beta), _p(out), _dt(x), x.numel() // C, C, eps, _stream())
 
     def attention(self, q, k, v, out, heads, scale, split=False):
         self._cuda(q, k, v)
@@ -246,10 +268,10 @@ class CudaBackend:
             o = out.buf if pair else out
             self._cuda(o)
             self._call("fb200_attention_split", _p(q), _pitch(q), _p(k), _pitch(k), _p(v), _pitch(v), _p(o), F16PAIR if pair else F32, _pitch(o), B, Lq, k.shape[1],
-                       heads, C // heads, ctypes.c_float(scale), _stream())
+                       heads, C // heads, scale, _stream())
             return
         self._call("fb200_attention", _p(q), _pitch(q), _p(k), _pitch(k), _p(v), _pitch(v), _p(out), _pitch(out), _dt(q), B, Lq, k.shape[1],
-                   heads, C // heads, ctypes.c_float(scale), _stream())
+                   heads, C // heads, scale, _stream())
 
     def msda(self, value, oa, ref, shapes, P, heads, out):
         self._cuda(value, oa, ref)
@@ -271,34 +293,34 @@ class CudaBackend:
         if gather is not None and valid is None:
             S = x.shape[-2]
         self._call("fb200_layernorm_ex", _p(x), _pitch(x), _p(res), _p(gather), 0 if gather is None else gather.shape[-1], _p(valid), S, _p(fill), _p(gamma), _p(beta),
-                   ctypes.c_float(eps), ctypes.c_int64(M), C, _p(out_f32), _p(None if out_pair is None else out_pair.buf), _p(pos),
-                   ctypes.c_int64(0 if pos is None else pos.numel() // C), _p(None if out_pair_pos is None else out_pair_pos.buf), _stream())
+                   eps, M, C, _p(out_f32), _p(None if out_pair is None else out_pair.buf), _p(pos),
+                   0 if pos is None else pos.numel() // C, _p(None if out_pair_pos is None else out_pair_pos.buf), _stream())
 
     def split_pair_ex(self, x, act, pos, out_pair, out_pair_pos):
         self._cuda(x)
         C = x.shape[-1]
-        self._call("fb200_split_pair_ex", _p(x), ctypes.c_int64(x.numel() // C), C, _pitch(x), act, _p(pos), ctypes.c_int64(0 if pos is None else pos.numel() // C),
+        self._call("fb200_split_pair_ex", _p(x), x.numel() // C, C, _pitch(x), act, _p(pos), 0 if pos is None else pos.numel() // C,
                    _p(None if out_pair is None else out_pair.buf), _p(None if out_pair_pos is None else out_pair_pos.buf), _stream())
 
     def box_refine_qpos(self, delta, ref_in, ref_out, w0, b0, qpos_pair):
         self._cuda(ref_in)
         self._call("fb200_box_refine_qpos", _p(delta), _p(ref_in), _p(ref_out), _p(w0), _p(b0), 0 if w0 is None else w0.shape[0],
-                   _p(None if qpos_pair is None else qpos_pair.buf), ctypes.c_int64(ref_in.numel() // 4), _stream())
+                   _p(None if qpos_pair is None else qpos_pair.buf), ref_in.numel() // 4, _stream())
 
     def sigmoid_rows(self, x, out):
         self._cuda(x, out)
         C = x.shape[-1]
-        self._call("fb200_sigmoid_rows", _p(x), _pitch(x), ctypes.c_int64(x.numel() // C), C, _p(out), _stream())
+        self._call("fb200_sigmoid_rows", _p(x), _pitch(x), x.numel() // C, C, _p(out), _stream())
 
     def row_select(self, x, valid, fill, out):
         self._cuda(x, valid, fill, out)
         C = x.shape[-1]
-        self._call("fb200_row_select", _p(x), _p(valid), _p(fill), _p(out), _dt(x), ctypes.c_int64(x.numel() // C), valid.numel(), C, _stream())
+        self._call("fb200_row_select", _p(x), _p(valid), _p(fill), _p(out), _dt(x), x.numel() // C, valid.numel(), C, _stream())
 
     def rowmax(self, x, out):
         self._cuda(x, out)
         N = x.shape[-1]
-        self._call("fb200_rowmax", _p(x), _dt(x), ctypes.c_int64(out.numel()), N, _pitch(x), _p(out), _stream())
+        self._call("fb200_rowmax", _p(x), _dt(x), out.numel(), N, _pitch(x), _p(out), _stream())
 
     def topk(self, x, K, out_idx, out_val):
         self._cuda(x, out_idx)
@@ -312,12 +334,12 @@ class CudaBackend:
 
     def box_op(self, mode, x, ref, idx, out):
         self._cuda(x, out)
-        self._call("fb200_box_op", mode, _p(x), _p(ref), _p(idx), _p(out), ctypes.c_int64(x.numel()), _stream())
+        self._call("fb200_box_op", mode, _p(x), _p(ref), _p(idx), _p(out), x.numel(), _stream())
 
     def detr_postprocess(self, scores, boxes, sizes, K, thr, out_scores, out_labels, out_boxes, out_query, out_count):
         self._cuda(scores, boxes, sizes)
         B, Q, C = scores.shape
-        self._call("fb200_detr_postprocess", _p(scores), _p(boxes), _p(sizes), B, Q, C, K, ctypes.c_float(thr), _p(out_scores), _p(out_labels),
+        self._call("fb200_detr_postprocess", _p(scores), _p(boxes), _p(sizes), B, Q, C, K, thr, _p(out_scores), _p(out_labels),
                    _p(out_boxes), _p(out_query), _p(out_count), _stream())
 
 
@@ -325,6 +347,256 @@ class CudaBackend:
         self._cuda(scores, boxes, sizes)
         B, Q, C = scores.shape
         self._call("fb200_detr_eval_postprocess", _p(scores), _p(boxes), _p(sizes), B, Q, C, K, _p(out_scores), _p(out_labels), _p(out_boxes), _p(out_count), _stream())
+
+    # ---- MaskFormer-family operators -------------------------------------------------------------------------
+    def upsample_nearest_add(self, y, cur, out):
+        self._cuda(y, cur, out)
+        B, h, w, C = y.shape
+        self._call("fb200_upsample_nearest_add", _p(y), _p(cur), _p(out), _dt(y), B, h, w, cur.shape[1], cur.shape[2], C, _stream())
+
+    def attn_mask_build(self, x, Q, mask, allowed):
+        self._cuda(x, mask, allowed)
+        B, h, w, Qp = x.shape
+        self._call("fb200_attn_mask_build", _p(x), _dt(x), B, h * w, Qp, Q, _p(mask), mask.shape[2], _p(allowed), _stream())
+
+    def attention_masked(self, q, k, v, mask, allowed, out, heads, scale):
+        self._cuda(q, k, v, mask, allowed, out)
+        B, Lq, C = q.shape
+        self._call("fb200_attention_masked", _p(q), _pitch(q), _p(k), _pitch(k), _p(v), _pitch(v), _p(mask), mask.shape[2], _p(allowed), _p(out), _pitch(out),
+                   _dt(q), B, Lq, k.shape[1], heads, C // heads, scale, _stream())
+
+    def attention_masked_split(self, q, k, v, mask, allowed, out, heads, scale):
+        """k / v: fp32 tensors [B,Lk,C] or `Pair`s (hi / lo fp16 planes written by their projection)"""
+        pair = isinstance(k, Pair)
+        kh, vh = (k.hi, v.hi) if pair else (k, v)
+        self._cuda(q, kh, vh, mask, allowed, out)
+        B, Lq, C = q.shape
+        self._call("fb200_attention_masked_split", _p(q), _pitch(q), _p(kh), _pitch(kh), _p(vh), _pitch(vh), F16PAIR if pair else F32, k.lo_off if pair else 0,
+                   _p(mask), mask.shape[2], _p(allowed), _p(out), _pitch(out), B, Lq, kh.shape[1], heads, C // heads, scale, _stream())
+
+    def softmax_drop_last(self, x, out):
+        self._cuda(x, out)
+        N = x.shape[-1]
+        self._call("fb200_softmax_drop_last", _p(x), x.numel() // N, N, _pitch(x), _p(out), _stream())
+
+    def mask_sigmoid_upsample(self, x, Q, out):
+        self._cuda(x, out)
+        B, h, w, Qp = x.shape
+        self._call("fb200_mask_sigmoid_upsample", _p(x), _dt(x), B, h, w, Qp, Q, _p(out), out.shape[2], out.shape[3], _stream())
+
+    def mask_sigmoid_upsample_argmax(self, x, Q, scores, labels, counts):
+        self._cuda(x, scores, labels, counts)
+        B, h, w, Qp = x.shape
+        self._call("fb200_mask_sigmoid_upsample_argmax", _p(x), _dt(x), B, h, w, Qp, Q, _p(scores), labels.shape[1], labels.shape[2], _p(labels), _p(counts), _stream())
+
+    def mask_sigmoid_upsample_stats(self, x, Q, size, thr, count, psum):
+        self._cuda(x, count, psum)
+        B, h, w, Qp = x.shape
+        self._call("fb200_mask_sigmoid_upsample_stats", _p(x), _dt(x), B, h, w, Qp, Q, size[0], size[1], thr, _p(count), _p(psum), _stream())
+
+    def mask_sigmoid_upsample_select(self, x, bq, out):
+        self._cuda(x, bq, out)
+        _, h, w, Qp = x.shape
+        self._call("fb200_mask_sigmoid_upsample_select", _p(x), _dt(x), h, w, Qp, _p(bq), bq.shape[0], _p(out), out.shape[1], out.shape[2], _stream())
+
+    def mask_stats(self, masks, thr, count, psum):
+        self._cuda(masks, count, psum)
+        B, Q, H, W = masks.shape
+        self._call("fb200_mask_stats", _p(masks), B * Q, H * W, thr, _p(count), _p(psum), _stream())
+
+    def mask_resize_bbox(self, masks, bq, thr, out_masks, out_bbox):
+        self._cuda(masks, bq, out_masks, out_bbox)
+        B, Q, H, W = masks.shape
+        self._call("fb200_mask_resize_bbox", _p(masks), Q, H, W, _p(bq), bq.shape[0], thr, _p(out_masks), out_masks.shape[1], out_masks.shape[2], _p(out_bbox), _stream())
+
+    # ---- BiSeNetFormer-family operators ----------------------------------------------------------------------
+    def dwconv3x3s2(self, x, w9c, scale, bias, out):
+        self._cuda(x, w9c, out)
+        B, H, W, C = x.shape
+        self._call("fb200_dwconv3x3s2_bn", _p(x), _dt(x), B, H, W, C, _p(w9c), _p(scale), _p(bias), _p(out), _stream())
+
+    def avgpool3x3s2(self, x, out):
+        self._cuda(x, out)
+        B, H, W, C = x.shape
+        self._call("fb200_avgpool3x3s2", _p(x), _dt(x), B, H, W, C, _p(out), _pitch(out), _stream())
+
+    def global_avgpool(self, x, out):
+        self._cuda(x, out)
+        B, C = x.shape[0], x.shape[-1]
+        self._call("fb200_global_avgpool", _p(x), _dt(x), B, x.numel() // (B * C), C, _p(out), _stream())
+
+    def channel_scale(self, x, gate, addvec, addt, self_add, out):
+        self._cuda(x, gate, out)
+        B, C = x.shape[0], x.shape[-1]
+        self._call("fb200_channel_scale", _p(x), _p(gate), _p(addvec), _p(addt), int(self_add), _p(out), _dt(x), B, x.numel() // (B * C), C, _stream())
+
+    def mask_argmax(self, masks, scores, labels, counts):
+        self._cuda(masks, scores, labels, counts)
+        B, Q, H, W = masks.shape
+        self._call("fb200_mask_argmax", _p(masks), _p(scores), B, Q, H * W, _p(labels), _p(counts), _stream())
+
+    def label_resize_bbox(self, labels, bq, out_masks, out_bbox):
+        self._cuda(labels, bq, out_masks, out_bbox)
+        self._call("fb200_label_resize_bbox", _p(labels), labels.shape[1], labels.shape[2], _p(bq), bq.shape[0], _p(out_masks), out_masks.shape[1], out_masks.shape[2],
+                   _p(out_bbox), _stream())
+
+    # ---- backward / training-mode operators (autograd_ops.py and the training graph) -------------------------
+    def conv_wgrad(self, x, dy, KH, KW, stride, pad, dw):
+        self._cuda(x, dy, dw)
+        B, H, W, Cin = x.shape
+        _, Ho, Wo, Cout = dy.shape
+        ws = _ws(self.lib.fb200_conv_wgrad_workspace_bytes(B, Ho, Wo, Cin, Cout, KH, KW), x.device)
+        self._call("fb200_conv_wgrad", _p(x), B, H, W, Cin, x.stride(2), _p(dy), Ho, Wo, Cout, dy.stride(2), KH, KW, stride, pad, _p(dw), 0, _p(ws), _stream())
+
+    def conv_wgrad_tc_supported(self, x_shape, dy_shape, KH, KW, stride, pad):
+        B, H, W, Cin = x_shape
+        _, Ho, Wo, Cout = dy_shape
+        return bool(self.lib.fb200_conv_wgrad_tc_supported(B, H, W, Cin, Ho, Wo, Cout, KH, KW, stride, pad))
+
+    def conv_wgrad_tc(self, x_pair, dy_pair, KH, KW, stride, pad, dw):
+        self._cuda(x_pair, dy_pair, dw)
+        B, H, W, C2 = x_pair.shape
+        Cin, Cout = C2 // 2, dy_pair.shape[-1] // 2
+        ws = _ws(self.lib.fb200_conv_wgrad_tc_workspace_bytes(B, dy_pair.shape[1], dy_pair.shape[2], Cin, Cout, KH, KW), x_pair.device)
+        self._call("fb200_conv_wgrad_tc", _p(x_pair), B, H, W, Cin, _p(dy_pair), Cout, KH, KW, stride, pad, _p(dw), 0, _p(ws), _stream())
+
+    def conv_wgrad_tc_f16(self, x16, dy16, KH, KW, stride, pad, dw):
+        self._cuda(x16, dy16, dw)
+        B, H, W, Cin = x16.shape
+        Cout = dy16.shape[-1]
+        ws = _ws(self.lib.fb200_conv_wgrad_tc_workspace_bytes(B, dy16.shape[1], dy16.shape[2], Cin, Cout, KH, KW), x16.device)
+        self._call("fb200_conv_wgrad_tc_f16", _p(x16), B, H, W, Cin, _p(dy16), Cout, KH, KW, stride, pad, _p(dw), 0, _p(ws), _stream())
+
+    def dilate2(self, dy, out):
+        self._cuda(dy, out)
+        B, Ho, Wo, C = dy.shape
+        self._call("fb200_dilate2", _p(dy), B, Ho, Wo, C, out.shape[1], out.shape[2], _p(out), _stream())
+
+    def _col_ws(self, C, device):
+        return _ws(self.lib.fb200_col_workspace_bytes(C), device)
+
+    def colsum(self, x2d, out):
+        self._cuda(x2d, out)
+        R, C = x2d.shape
+        self._call("fb200_colsum", _p(x2d), R, C, x2d.stride(0), _p(out), 0, _p(self._col_ws(C, x2d.device)), _stream())
+
+    def bn_train_fwd(self, x2d, gamma, beta, res2d, act, eps, momentum, rmean, rvar, save_mean, save_rstd, y2d):
+        self._cuda(x2d, gamma, beta, y2d)
+        R, C = x2d.shape
+        self._call("fb200_bn_train_fwd", _p(x2d), x2d.stride(0), R, C, _p(gamma), _p(beta), _p(res2d), 0 if res2d is None else res2d.stride(0), act, eps,
+                   momentum, _p(rmean), _p(rvar), _p(save_mean), _p(save_rstd), _p(y2d), y2d.stride(0), _p(self._col_ws(C, x2d.device)), _stream())
+
+    def bn_train_bwd(self, x2d, dy2d, y2d, gamma, beta, save_mean, save_rstd, act, dx2d, dres2d, dgamma, dbeta):
+        self._cuda(x2d, dy2d, dx2d)
+        R, C = x2d.shape
+        self._call("fb200_bn_train_bwd", _p(x2d), x2d.stride(0), _p(dy2d), dy2d.stride(0), _p(y2d), 0 if y2d is None else y2d.stride(0), R, C, _p(gamma), _p(beta),
+                   _p(save_mean), _p(save_rstd), act, _p(dx2d), dx2d.stride(0), _p(dres2d), 0 if dres2d is None else dres2d.stride(0), _p(dgamma), _p(dbeta), 0,
+                   _p(self._col_ws(C, x2d.device)), _stream())
+
+    def bn_stats(self, x2d, mean, var):
+        self._cuda(x2d, mean, var)
+        R, C = x2d.shape
+        self._call("fb200_bn_stats", _p(x2d), x2d.stride(0), R, C, _p(mean), _p(var), _p(self._col_ws(C, x2d.device)), _stream())
+
+    def bn_sync_combine(self, allst, eps, momentum, rmean, rvar, mean, rstd, inv_total):
+        self._cuda(allst, mean, rstd, inv_total)
+        world, width = allst.shape
+        self._call("fb200_bn_sync_combine", _p(allst), world, (width - 1) // 2, eps, momentum, _p(rmean), _p(rvar), _p(mean), _p(rstd), _p(inv_total), _stream())
+
+    def bn_apply(self, x2d, mean, rstd, gamma, beta, res2d, act, y2d):
+        self._cuda(x2d, mean, rstd, gamma, beta, y2d)
+        R, C = x2d.shape
+        self._call("fb200_bn_apply", _p(x2d), x2d.stride(0), R, C, _p(mean), _p(rstd), _p(gamma), _p(beta), _p(res2d), 0 if res2d is None else res2d.stride(0), act,
+                   _p(y2d), y2d.stride(0), _stream())
+
+    def bn_bwd_reduce(self, x2d, dy2d, y2d, gamma, beta, mean, rstd, act, sum_dy, sum_dy_xhat):
+        self._cuda(x2d, dy2d, sum_dy, sum_dy_xhat)
+        R, C = x2d.shape
+        self._call("fb200_bn_bwd_reduce", _p(x2d), x2d.stride(0), _p(dy2d), dy2d.stride(0), _p(y2d), 0 if y2d is None else y2d.stride(0), R, C, _p(gamma), _p(beta),
+                   _p(mean), _p(rstd), act, _p(sum_dy), _p(sum_dy_xhat), _p(self._col_ws(C, x2d.device)), _stream())
+
+    def bn_bwd_apply(self, x2d, dy2d, y2d, gamma, beta, mean, rstd, sum_dy, sum_dy_xhat, inv_count, act, dx2d, dres2d):
+        self._cuda(x2d, dy2d, dx2d)
+        R, C = x2d.shape
+        self._call("fb200_bn_bwd_apply", _p(x2d), x2d.stride(0), _p(dy2d), dy2d.stride(0), _p(y2d), 0 if y2d is None else y2d.stride(0), R, C, _p(gamma), _p(beta),
+                   _p(mean), _p(rstd), _p(sum_dy), _p(sum_dy_xhat), inv_count, act, _p(dx2d), dx2d.stride(0), _p(dres2d), 0 if dres2d is None else dres2d.stride(0), _stream())
+
+    def add_act(self, a, b, dy, act, out):
+        self._cuda(a, out)
+        self._call("fb200_add_act", _p(a), _p(b), _p(dy), act, a.numel(), _p(out), _stream())
+
+    def maxpool_bwd(self, x, dy, dx):
+        self._cuda(x, dy, dx)
+        B, H, W, C = x.shape
+        self._call("fb200_maxpool3x3s2_bwd", _p(x), _p(dy), B, H, W, C, _p(dx), _stream())
+
+    def avgpool_bwd(self, dy, dx):
+        self._cuda(dy, dx)
+        B, H, W, C = dx.shape
+        self._call("fb200_avgpool2x2_ceil_bwd", _p(dy), B, H, W, C, _p(dx), _stream())
+
+    def resize_bwd(self, dy, dx):
+        self._cuda(dy, dx)
+        B, H, W, C = dx.shape
+        self._call("fb200_resize_bilinear_bwd", _p(dy), dy.stride(2), B, H, W, C, dy.shape[1], dy.shape[2], _p(dx), _stream())
+
+    def layernorm_bwd(self, x2d, res2d, gamma, dy2d, eps, dx2d, dgamma, dbeta):
+        self._cuda(x2d, dy2d, dx2d)
+        M, C = x2d.shape
+        self._call("fb200_layernorm_bwd", _p(x2d), _p(res2d), _p(gamma), _p(dy2d), M, C, eps, _p(dx2d), _p(dgamma), _p(dbeta), 0,
+                   _p(self._col_ws(C, x2d.device)), _stream())
+
+    def attention_bwd(self, q, k, v, o, do, heads, scale, dq, dk, dv):
+        self._cuda(q, k, v, o, do, dq, dk, dv)
+        B, Lq, C = q.shape
+        self._call("fb200_attention_bwd", _p(q), q.stride(1), _p(k), k.stride(1), _p(v), v.stride(1), _p(o), o.stride(1), _p(do), do.stride(1), B, Lq, k.shape[1], heads,
+                   C // heads, scale, _p(dq), dq.stride(1), _p(dk), dk.stride(1), _p(dv), dv.stride(1), _stream())
+
+    def msda_bwd(self, value, oa, ref, do, shapes, P, heads, dvalue, doa):
+        self._cuda(value, oa, ref, do, dvalue, doa)
+        B, S, _ = value.shape
+        Q = oa.shape[1]
+        arr = (ctypes.c_int * (2 * len(shapes)))(*[int(v) for hw in shapes for v in hw])
+        self._call("fb200_msda_bwd", _p(value), value.stride(1), _p(oa), oa.stride(1), _p(ref), _p(do), do.stride(1), arr, len(shapes), P, B, S, Q, heads, _p(dvalue),
+                   dvalue.stride(1), _p(doa), doa.stride(1), _stream())
+
+    # ---- DETR training criterion (criterion.py) --------------------------------------------------------------
+    def detr_match_cost(self, logits, boxes, tl, tb, toff, wts, alpha, gamma, cost):
+        self._cuda(logits, boxes, tl, tb, toff, cost)
+        L, B, Q, C = logits.shape
+        self._call("fb200_detr_match_cost", _p(logits), _p(boxes), _p(tl), _p(tb), _p(toff), L, B, Q, C, tl.shape[0],
+                   wts[0], wts[1], wts[2], alpha, gamma, _p(cost), _stream())
+
+    def hungarian(self, cost, toff, B, max_targets, match_q):
+        self._cuda(cost, toff, match_q)
+        L, T, Q = cost.shape
+        self._call("fb200_hungarian", _p(cost), _p(toff), L, B, Q, T, max_targets, _p(match_q), _stream())
+
+    def detr_loss(self, logits, boxes, tl, tb, toff, match_q, num_boxes, wts, alpha, gamma, losses, g_logits, g_l1, g_giou):
+        self._cuda(logits, boxes, toff, losses, g_logits, g_l1, g_giou)
+        L, B, Q, C = logits.shape
+        ws = _ws(self.lib.fb200_detr_loss_workspace_bytes(L, B, Q), logits.device)
+        self._call("fb200_detr_loss", _p(logits), _p(boxes), _p(tl), _p(tb), _p(toff), _p(match_q), L, B, Q, C, 0 if tl is None else tl.shape[0],
+                   num_boxes, wts[0], wts[1], wts[2], alpha, gamma,
+                   _p(losses), _p(g_logits), _p(g_l1), _p(g_giou), _p(ws), _stream())
+
+    # ---- optimiser step (train_step.py) ----------------------------------------------------------------------
+    def optim_workspace(self, device):
+        return torch.zeros(int(self.lib.fb200_optim_workspace_bytes()), dtype=torch.uint8, device=device)
+
+    def grad_stats(self, grads, ws):
+        self._cuda(grads, ws)
+        self._call("fb200_grad_stats", _p(grads), grads.numel(), _p(ws), _stream())
+
+    def optim_finalize(self, ws, ctrl, max_norm, clip_passes, inv_world, use_scaler, growth, backoff, growth_interval, beta1, beta2):
+        self._cuda(ws, ctrl)
+        self._call("fb200_optim_finalize", _p(ws), _p(ctrl), max_norm, int(clip_passes), inv_world, int(use_scaler),
+                   growth, backoff, int(growth_interval), beta1, beta2, _stream())
+
+    def adamw_step(self, params, grads, m, v, chunk_start, chunk_len, chunk_seg, seg_lr, seg_wd, seg_active, lr_factor, beta1, beta2, eps, ctrl):
+        self._cuda(params, grads, m, v, chunk_start, chunk_len, chunk_seg, seg_lr, seg_wd, ctrl)
+        self._call("fb200_adamw_step", _p(params), _p(grads), _p(m), _p(v), _p(chunk_start), _p(chunk_len), _p(chunk_seg), chunk_len.shape[0], _p(seg_lr), _p(seg_wd), _p(seg_active),
+                   lr_factor, beta1, beta2, eps, _p(ctrl), _stream())
 
 
 class Pair:
@@ -817,88 +1089,6 @@ except Exception:  # pragma: no cover - e.g. double import under a different mod
 # ------------------------------------------------------------------------------------------------
 # MaskFormer-family operators (SURVEY §8 rows a14-a17)
 # ------------------------------------------------------------------------------------------------
-EXPORTED_SYMBOLS = EXPORTED_SYMBOLS + (
-    "fb200_upsample_nearest_add", "fb200_attn_mask_build", "fb200_attention_masked", "fb200_attention_masked_split", "fb200_softmax_drop_last",
-    "fb200_mask_sigmoid_upsample", "fb200_mask_sigmoid_upsample_argmax", "fb200_mask_sigmoid_upsample_stats", "fb200_mask_sigmoid_upsample_select", "fb200_mask_stats", "fb200_mask_resize_bbox",
-)
-
-
-def _cb_upsample_nearest_add(self, y, cur, out):
-    self._cuda(y, cur, out)
-    B, h, w, C = y.shape
-    self._call("fb200_upsample_nearest_add", _p(y), _p(cur), _p(out), _dt(y), B, h, w, cur.shape[1], cur.shape[2], C, _stream())
-
-
-def _cb_attn_mask_build(self, x, Q, mask, allowed):
-    self._cuda(x, mask, allowed)
-    B, h, w, Qp = x.shape
-    self._call("fb200_attn_mask_build", _p(x), _dt(x), B, h * w, Qp, Q, _p(mask), mask.shape[2], _p(allowed), _stream())
-
-
-def _cb_attention_masked(self, q, k, v, mask, allowed, out, heads, scale):
-    self._cuda(q, k, v, mask, allowed, out)
-    B, Lq, C = q.shape
-    self._call("fb200_attention_masked", _p(q), _pitch(q), _p(k), _pitch(k), _p(v), _pitch(v), _p(mask), mask.shape[2], _p(allowed), _p(out), _pitch(out),
-               _dt(q), B, Lq, k.shape[1], heads, C // heads, ctypes.c_float(scale), _stream())
-
-
-def _cb_attention_masked_split(self, q, k, v, mask, allowed, out, heads, scale):
-    """k / v: fp32 tensors [B,Lk,C] or `Pair`s (hi / lo fp16 planes written by their projection)"""
-    pair = isinstance(k, Pair)
-    kh, vh = (k.hi, v.hi) if pair else (k, v)
-    self._cuda(q, kh, vh, mask, allowed, out)
-    B, Lq, C = q.shape
-    self._call("fb200_attention_masked_split", _p(q), _pitch(q), _p(kh), _pitch(kh), _p(vh), _pitch(vh), F16PAIR if pair else F32, ctypes.c_int64(k.lo_off if pair else 0),
-               _p(mask), mask.shape[2], _p(allowed), _p(out), _pitch(out), B, Lq, kh.shape[1], heads, C // heads, ctypes.c_float(scale), _stream())
-
-
-def _cb_softmax_drop_last(self, x, out):
-    self._cuda(x, out)
-    N = x.shape[-1]
-    self._call("fb200_softmax_drop_last", _p(x), ctypes.c_int64(x.numel() // N), N, _pitch(x), _p(out), _stream())
-
-
-def _cb_mask_sigmoid_upsample(self, x, Q, out):
-    self._cuda(x, out)
-    B, h, w, Qp = x.shape
-    self._call("fb200_mask_sigmoid_upsample", _p(x), _dt(x), B, h, w, Qp, Q, _p(out), out.shape[2], out.shape[3], _stream())
-
-
-def _cb_mask_sigmoid_upsample_argmax(self, x, Q, scores, labels, counts):
-    self._cuda(x, scores, labels, counts)
-    B, h, w, Qp = x.shape
-    self._call("fb200_mask_sigmoid_upsample_argmax", _p(x), _dt(x), B, h, w, Qp, Q, _p(scores), labels.shape[1], labels.shape[2], _p(labels), _p(counts), _stream())
-
-
-def _cb_mask_sigmoid_upsample_stats(self, x, Q, size, thr, count, psum):
-    self._cuda(x, count, psum)
-    B, h, w, Qp = x.shape
-    self._call("fb200_mask_sigmoid_upsample_stats", _p(x), _dt(x), B, h, w, Qp, Q, size[0], size[1], ctypes.c_float(thr), _p(count), _p(psum), _stream())
-
-
-def _cb_mask_sigmoid_upsample_select(self, x, bq, out):
-    self._cuda(x, bq, out)
-    _, h, w, Qp = x.shape
-    self._call("fb200_mask_sigmoid_upsample_select", _p(x), _dt(x), h, w, Qp, _p(bq), bq.shape[0], _p(out), out.shape[1], out.shape[2], _stream())
-
-
-def _cb_mask_stats(self, masks, thr, count, psum):
-    self._cuda(masks, count, psum)
-    B, Q, H, W = masks.shape
-    self._call("fb200_mask_stats", _p(masks), ctypes.c_int64(B * Q), ctypes.c_int64(H * W), ctypes.c_float(thr), _p(count), _p(psum), _stream())
-
-
-def _cb_mask_resize_bbox(self, masks, bq, thr, out_masks, out_bbox):
-    self._cuda(masks, bq, out_masks, out_bbox)
-    B, Q, H, W = masks.shape
-    self._call("fb200_mask_resize_bbox", _p(masks), Q, H, W, _p(bq), bq.shape[0], ctypes.c_float(thr), _p(out_masks), out_masks.shape[1], out_masks.shape[2], _p(out_bbox), _stream())
-
-
-for _n, _f in (("mask_sigmoid_upsample_stats", _cb_mask_sigmoid_upsample_stats), ("mask_sigmoid_upsample_select", _cb_mask_sigmoid_upsample_select),
-               ("mask_sigmoid_upsample_argmax", _cb_mask_sigmoid_upsample_argmax), ("upsample_nearest_add", _cb_upsample_nearest_add), ("attn_mask_build", _cb_attn_mask_build), ("attention_masked", _cb_attention_masked), ("attention_masked_split", _cb_attention_masked_split),
-               ("softmax_drop_last", _cb_softmax_drop_last), ("mask_sigmoid_upsample", _cb_mask_sigmoid_upsample), ("mask_stats", _cb_mask_stats),
-               ("mask_resize_bbox", _cb_mask_resize_bbox)):
-    setattr(CudaBackend, _n, _f)
 
 
 def upsample_nearest_add(y, cur):
@@ -1002,49 +1192,6 @@ def mask_resize_bbox(masks, bq_i32, thr: float, size):
 # BiSeNetFormer-family operators (SURVEY §8 rows a18-a19)
 # ------------------------------------------------------------------------------------------------
 ACT_SIGMOID = 4
-EXPORTED_SYMBOLS = EXPORTED_SYMBOLS + ("fb200_dwconv3x3s2_bn", "fb200_avgpool3x3s2", "fb200_global_avgpool", "fb200_channel_scale", "fb200_mask_argmax",
-                                       "fb200_label_resize_bbox")
-
-
-def _cb_dwconv3x3s2(self, x, w9c, scale, bias, out):
-    self._cuda(x, w9c, out)
-    B, H, W, C = x.shape
-    self._call("fb200_dwconv3x3s2_bn", _p(x), _dt(x), B, H, W, C, _p(w9c), _p(scale), _p(bias), _p(out), _stream())
-
-
-def _cb_avgpool3x3s2(self, x, out):
-    self._cuda(x, out)
-    B, H, W, C = x.shape
-    self._call("fb200_avgpool3x3s2", _p(x), _dt(x), B, H, W, C, _p(out), _pitch(out), _stream())
-
-
-def _cb_global_avgpool(self, x, out):
-    self._cuda(x, out)
-    B, C = x.shape[0], x.shape[-1]
-    self._call("fb200_global_avgpool", _p(x), _dt(x), B, x.numel() // (B * C), C, _p(out), _stream())
-
-
-def _cb_channel_scale(self, x, gate, addvec, addt, self_add, out):
-    self._cuda(x, gate, out)
-    B, C = x.shape[0], x.shape[-1]
-    self._call("fb200_channel_scale", _p(x), _p(gate), _p(addvec), _p(addt), int(self_add), _p(out), _dt(x), B, ctypes.c_int64(x.numel() // (B * C)), C, _stream())
-
-
-def _cb_mask_argmax(self, masks, scores, labels, counts):
-    self._cuda(masks, scores, labels, counts)
-    B, Q, H, W = masks.shape
-    self._call("fb200_mask_argmax", _p(masks), _p(scores), B, Q, ctypes.c_int64(H * W), _p(labels), _p(counts), _stream())
-
-
-def _cb_label_resize_bbox(self, labels, bq, out_masks, out_bbox):
-    self._cuda(labels, bq, out_masks, out_bbox)
-    self._call("fb200_label_resize_bbox", _p(labels), labels.shape[1], labels.shape[2], _p(bq), bq.shape[0], _p(out_masks), out_masks.shape[1], out_masks.shape[2],
-               _p(out_bbox), _stream())
-
-
-for _n, _f in (("dwconv3x3s2", _cb_dwconv3x3s2), ("avgpool3x3s2", _cb_avgpool3x3s2), ("global_avgpool", _cb_global_avgpool), ("channel_scale", _cb_channel_scale),
-               ("mask_argmax", _cb_mask_argmax), ("label_resize_bbox", _cb_label_resize_bbox)):
-    setattr(CudaBackend, _n, _f)
 
 
 def dwconv3x3s2(x, w9c, scale, bias):

@@ -12,7 +12,6 @@ bucket by bucket (reverse parameter order, as the backward pass produces them) f
 """
 from __future__ import annotations
 
-import ctypes
 from typing import Dict, Iterable, List, Optional, Sequence
 
 import torch
@@ -20,39 +19,9 @@ import torch.distributed as dist
 import torch.nn as nn
 
 from . import ops
-from .ops import CudaBackend, _p, _stream
-
-ops.EXPORTED_SYMBOLS = ops.EXPORTED_SYMBOLS + ("fb200_optim_workspace_bytes", "fb200_grad_stats", "fb200_optim_finalize", "fb200_adamw_step")
 
 CTRL_SCALE, CTRL_GROWTH_TRACKER, CTRL_FOUND_INF, CTRL_GRAD_NORM, CTRL_GMUL, CTRL_STEP, CTRL_BC1, CTRL_BC2_SQRT, CTRL_CLIP_COEF = range(9)
 CTRL_WORDS = 16
-
-
-# ---- backend methods ------------------------------------------------------------------------------------------
-def _cb_optim_workspace(self, device):
-    self.lib.fb200_optim_workspace_bytes.restype = ctypes.c_int64
-    return torch.zeros(int(self.lib.fb200_optim_workspace_bytes()), dtype=torch.uint8, device=device)
-
-
-def _cb_grad_stats(self, grads, ws):
-    self._cuda(grads, ws)
-    self._call("fb200_grad_stats", _p(grads), ctypes.c_int64(grads.numel()), _p(ws), _stream())
-
-
-def _cb_optim_finalize(self, ws, ctrl, max_norm, clip_passes, inv_world, use_scaler, growth, backoff, growth_interval, beta1, beta2):
-    self._cuda(ws, ctrl)
-    self._call("fb200_optim_finalize", _p(ws), _p(ctrl), ctypes.c_float(max_norm), int(clip_passes), ctypes.c_float(inv_world), int(use_scaler),
-               ctypes.c_float(growth), ctypes.c_float(backoff), int(growth_interval), ctypes.c_float(beta1), ctypes.c_float(beta2), _stream())
-
-
-def _cb_adamw_step(self, params, grads, m, v, chunk_start, chunk_len, chunk_seg, seg_lr, seg_wd, seg_active, lr_factor, beta1, beta2, eps, ctrl):
-    self._cuda(params, grads, m, v, chunk_start, chunk_len, chunk_seg, seg_lr, seg_wd, ctrl)
-    self._call("fb200_adamw_step", _p(params), _p(grads), _p(m), _p(v), _p(chunk_start), _p(chunk_len), _p(chunk_seg), chunk_len.shape[0], _p(seg_lr), _p(seg_wd), _p(seg_active),
-               ctypes.c_float(lr_factor), ctypes.c_float(beta1), ctypes.c_float(beta2), ctypes.c_float(eps), _p(ctrl), _stream())
-
-
-for _n, _f in (("optim_workspace", _cb_optim_workspace), ("grad_stats", _cb_grad_stats), ("optim_finalize", _cb_optim_finalize), ("adamw_step", _cb_adamw_step)):
-    setattr(CudaBackend, _n, _f)
 
 _NORM_TYPES = (nn.BatchNorm1d, nn.BatchNorm2d, nn.BatchNorm3d, nn.SyncBatchNorm, nn.GroupNorm, nn.InstanceNorm1d, nn.InstanceNorm2d, nn.InstanceNorm3d,
                nn.LayerNorm, nn.LocalResponseNorm)
